@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Benchmark of the HandyRL learner hot path on B200 (contract: see the task statement / DESIGN.md section 6).
+"""Benchmark of the HandyRL learner hot path on B200 (DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one learner step on one replay batch: Batcher output -> net forward -> fused loss
@@ -22,6 +22,9 @@ metric = learner samples/s = B*T*steps/s over all GPUs (BASELINE.json).
   cpu_baseline / --impl reference: the eager-PyTorch CPU port of the reference learner step (oracle/torch_learner.py,
                pinned to the reference's golden vectors) on the host cores: ALWAYS the workload's full batch, a fixed
                thread count, 3+ warm-ups, min / median / mean, loss-only and full step reported separately.
+
+--dump-outputs DIR writes what the last timed step of `value` handed back -- its six loss sums and the model state --
+as DIR/<name>.npy; the inputs depend on the arguments only, so two builds run with the same arguments can be compared.
 """
 import argparse
 import json
@@ -64,6 +67,7 @@ WORKLOADS = {
                       desc='configs[4] per-GPU shard: 64x64 obs / 512 actions, T=64 B=512/GPU P=2 Pa=1'),
 }
 L2_BYTES = 126e6
+DUMP_BYTES = 64 << 20
 CPU_THREADS = max(1, min(64, (os.cpu_count() or 2) // 2))       # fixed: the host's physical cores, at most 64
 
 
@@ -252,6 +256,22 @@ def reference_arm(opt, w):
 
 
 # ------------------------------------------------------------------------------ B200 arm
+
+def dump_outputs(path, stepper):
+    """The last step's loss sums (p, v, r, ent, total, dcnt) as losses.npy and every entry of the model's state_dict
+    after it as state.<key>.npy; float32 stays float32, everything else is written as float64."""
+    import numpy as np
+    stepper.stream.synchronize()
+    arrays = {'losses': stepper.last_losses.cpu()}
+    arrays.update(('state.' + k, v) for k, v in stepper.cpu_state_dict().items())
+    arrays = {k: (t if t.dtype == torch.float32 else t.double()).numpy() for k, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit('bench.py: --dump-outputs would write %d bytes (limit %d)' % (total, DUMP_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + '.npy'), a)
+
 
 def loss_kernel_name(A):
     """Which variant hrl_loss_fwd_bwd dispatches to for this action count (csrc/loss_kernel.cu)."""
@@ -502,6 +522,8 @@ def b200_arm(opt, w):
         ms, wall, per_rank_value = timed(lambda i: stepper.step_resident(dev_ring[i % R]), warm, opt.steps)
     kernel_ms, n_k = stepper.loss_kernel_ms()
     value = B * T * world * opt.steps / (ms * 1e-3)
+    if opt.dump_outputs and rank == 0:
+        dump_outputs(opt.dump_outputs, stepper)
 
     # ---- e2e: host batches, H2D inside (copy stream, one step ahead), loss read back every step (lagged by one step)
     pending = []
@@ -630,7 +652,7 @@ def b200_arm(opt, w):
         try:
             import contextlib
             with contextlib.redirect_stdout(sys.stderr):        # the Trainer prints the reference's progress lines
-                line['e2e_trainer'] = trainer_leg(w, steps=max(200, min(opt.steps, 2000)))
+                line['e2e_trainer'] = trainer_leg(w, steps=opt.steps)
         except Exception as e:  # noqa: BLE001
             line['e2e_trainer'] = {'error': '%s: %s' % (type(e).__name__, e)}
     if world == 1 and not opt.no_cpu and not opt.quick:
@@ -673,7 +695,12 @@ def main():
     ap.add_argument('--no-trainer', action='store_true', help='skip the Trainer (e2e_trainer) leg')
     ap.add_argument('--quick', action='store_true', help='value and e2e only')
     ap.add_argument('--cpu-budget-s', type=int, default=240, help='time box of --impl reference (steps are dropped, never the batch)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the last timed step\'s loss sums and model state to DIR/<name>.npy')
     opt = ap.parse_args()
+    if opt.steps < 1:
+        ap.error('--steps must be at least 1')
+    if opt.dump_outputs and opt.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
     w = WORKLOADS[opt.workload]
     if opt.impl == 'reference':
         reference_arm(opt, w)

@@ -1,22 +1,27 @@
-"""End to end: the REFERENCE's Learner, worker processes and server loop on top of handyrl_b200's Trainer.
+"""End to end: the reference's Learner, worker processes and server loop on top of handyrl_b200's Trainer.
 
     python tests/e2e_reference_learner.py [--uniform-net] [--epochs N]
 
-Needs the reference checkout (HANDYRL_REFERENCE, default /root/reference) -- it is NOT copied into this repo, so
-this script only runs where it is mounted.  With a CUDA device it trains the reference's own TicTacToe net through
-the GPU learner; with `--uniform-net` (no GPU needed) the environment's net is replaced by a parameter-free model, which
-exercises everything around the optimiser step: install(), Learner.feed_episodes -> Trainer.episodes, the trainer
-thread protocol, update() hand-offs, pickling the returned model for the workers and the workers unpickling it.
+With HANDYRL_REFERENCE naming a checkout of the original HandyRL (it is NOT part of this repo), that project's own
+Learner, workers and server run.  Without one, a stand-in `handyrl` package drives the Trainer through the same
+protocol (see StandInLearner).  With a CUDA device it trains a TicTacToe net through the GPU learner; with
+`--uniform-net` (no GPU needed) the net is replaced by a parameter-free model, which exercises everything around the
+optimiser step: install(), Learner.feed_episodes -> Trainer.episodes, the trainer thread protocol, update()
+hand-offs, pickling the returned model for the workers and the workers unpickling it.
 Prints E2E_OK on success.
 """
 import argparse
+import copy
 import os
+import pickle
 import sys
 import tempfile
+import threading
 
-REF = os.environ.get('HANDYRL_REFERENCE', '/root/reference')
+REF = os.environ.get('HANDYRL_REFERENCE')
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, REF)
+if REF:
+    sys.path.insert(0, REF)
 sys.path.insert(0, ROOT)
 
 
@@ -30,20 +35,109 @@ class UniformNet(torch.nn.Module):
         return {'policy': torch.zeros(x.shape[0], 9), 'value': torch.zeros(x.shape[0], 1)}
 
 
+def stand_in_worker(conn, wid):
+    """A worker process of StandInLearner: fetch the pickled model, run it, ship TicTacToe episodes in the reference's
+    wire format; ends when the learner closes the connection."""
+    from handyrl_b200.synthetic import tictactoe_episodes
+    rounds = 0
+    try:
+        while True:
+            conn.send(('model', None))
+            model = pickle.loads(conn.recv())
+            with torch.no_grad():
+                assert model(torch.zeros(2, 3, 3, 3))['policy'].shape == (2, 9)
+            conn.send(('episode', tictactoe_episodes(10, seed=1000 * wid + rounds)))
+            conn.recv()
+            rounds += 1
+    except (EOFError, OSError):
+        pass
+
+
+class StandInLearner:
+    """What the reference Learner does with its Trainer (train.py:403-630), for where no checkout of it is at hand: the
+    Trainer is built through the module attribute `Trainer(args, copy.deepcopy(self.model))`, its run() goes on a
+    thread, the server loop hands the model pickled to worker processes and feeds the episodes they return into
+    trainer.episodes (oldest dropped beyond maximum_episodes), and every update_episodes returned episodes after
+    minimum_episodes it calls trainer.update() and saves models/<epoch>.pth, until `epochs` epochs are done."""
+
+    def __init__(self, args, net=None):
+        import handyrl.train as module
+        self.args = args['train_args']
+        self.model = net
+        self.model_epoch = 0
+        self.num_returned_episodes = 0
+        self.trainer = module.Trainer(self.args, copy.deepcopy(self.model))
+
+    def update(self):
+        model, steps = self.trainer.update()
+        print('updated model(%d)' % steps)
+        self.model_epoch += 1
+        self.model = model if model is not None else self.model
+        os.makedirs('models', exist_ok=True)
+        torch.save(self.model.state_dict(), os.path.join('models', '%d.pth' % self.model_epoch))
+
+    def feed_episodes(self, episodes):
+        self.num_returned_episodes += len(episodes)
+        self.trainer.episodes.extend(episodes)
+        while len(self.trainer.episodes) > self.args['maximum_episodes']:
+            self.trainer.episodes.popleft()
+
+    def run(self):
+        import multiprocessing as mp
+        from multiprocessing.connection import wait
+        threading.Thread(target=self.trainer.run, daemon=True).start()
+        ctx = mp.get_context('spawn')
+        conns, procs = [], []
+        for wid in range(self.args['worker']['num_parallel']):
+            mine, theirs = ctx.Pipe()
+            procs.append(ctx.Process(target=stand_in_worker, args=(theirs, wid), daemon=True))
+            procs[-1].start()
+            theirs.close()
+            conns.append(mine)
+        next_update = self.args['minimum_episodes'] + self.args['update_episodes']
+        while self.model_epoch < self.args['epochs']:
+            for conn in wait(conns):
+                req, data = conn.recv()
+                if req == 'model':
+                    conn.send(pickle.dumps(self.model))
+                else:
+                    self.feed_episodes(data)
+                    conn.send(None)
+            if self.num_returned_episodes >= next_update:
+                next_update += self.args['update_episodes']
+                self.update()
+        for conn in conns:
+            conn.close()
+        for p in procs:
+            p.join(timeout=30)
+
+
+def install_stand_in():
+    """A stand-in `handyrl` package: the module attributes install() replaces, and StandInLearner."""
+    import types
+    train = types.ModuleType('handyrl.train')
+    for k in ('Trainer', 'Batcher', 'make_batch', 'forward_prediction', 'compute_loss'):
+        setattr(train, k, None)
+    train.Learner = StandInLearner
+    losses = types.ModuleType('handyrl.losses')
+    losses.compute_target = None
+    pkg = types.ModuleType('handyrl')
+    pkg.train, pkg.losses = train, losses
+    sys.modules.update({'handyrl': pkg, 'handyrl.train': train, 'handyrl.losses': losses})
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--uniform-net', action='store_true')
     ap.add_argument('--epochs', type=int, default=2)
     opt = ap.parse_args()
     os.chdir(tempfile.mkdtemp(prefix='hrl_e2e_'))           # the Learner writes models/<epoch>.pth into the cwd
+    if not REF:
+        install_stand_in()
 
     import handyrl_b200.train as b200
     ref = b200.install()                                       # the three lines INTEGRATION.md adds to main.py
     assert ref.Trainer is b200.Trainer
-
-    if opt.uniform_net:
-        import handyrl.envs.tictactoe as ttt
-        ttt.Environment.net = lambda self: UniformNet()
 
     args = {
         'env_args': {'env': 'TicTacToe'},
@@ -57,9 +151,16 @@ def main():
         },
         'worker_args': {'server_address': '', 'num_parallel': 2},
     }
-    from handyrl.environment import prepare_env
-    prepare_env(args['env_args'])
-    learner = ref.Learner(args=args)
+    if REF:
+        if opt.uniform_net:
+            import handyrl.envs.tictactoe as ttt
+            ttt.Environment.net = lambda self: UniformNet()
+        from handyrl.environment import prepare_env
+        prepare_env(args['env_args'])
+        learner = ref.Learner(args=args)
+    else:
+        from handyrl_b200.nets import tictactoe_net
+        learner = ref.Learner(args=args, net=UniformNet() if opt.uniform_net else tictactoe_net())
     assert isinstance(learner.trainer, b200.Trainer)
     learner.run()
     assert learner.model_epoch >= opt.epochs, learner.model_epoch

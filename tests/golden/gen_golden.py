@@ -12,6 +12,7 @@ Outputs (committed):
     tests/golden/rnn_cases.pkl      recurrent forward_prediction + compute_loss + parameter gradients (train.py:147-174)
     tests/golden/net_step_cases.pkl 3 optimiser steps of the reference's GeisterNet (DRC ConvLSTM, recurrent path) and
                                     GeeseNet (torus convolutions; `kaggle_environments` stubbed, SURVEY.md 8c)
+    tests/golden/generator_cases.pkl one self-play episode from the reference's Generator (generation.py:20-93)
 
 The reference has no golden vectors of its own for this path (SURVEY.md 8c), so the
 vectors are the reference's own outputs.  The fp64 quirk of `selected_prob` is avoided by
@@ -360,10 +361,26 @@ def gen_net_step_cases():
     print('net step cases:', list(out))
 
 
+def gen_generator_cases():
+    """One TicTacToe episode as the reference's Generator.generate returns it (generation.py:20-93): what a worker
+    ships, and what wire.install_worker_hook wraps."""
+    env_args = {'env': 'TicTacToe'}
+    prepare_env(env_args)
+    env = make_env(env_args)
+    torch.manual_seed(3)
+    model = ModelWrapper(env.net())
+    random.seed(3)
+    args = {'gamma': 0.8, 'compress_steps': 4}
+    ep = Generator(env, args).generate({p: model for p in env.players()}, {'player': env.players(), 'model_id': {}})
+    with open(os.path.join(HERE, 'generator_cases.pkl'), 'wb') as f:
+        pickle.dump({'tictactoe': {'args': args, 'episode': ep}}, f)
+    print('generator cases: tictactoe, %d steps' % ep['steps'])
+
+
 if __name__ == '__main__':
     os.chdir('/tmp')
-    if len(sys.argv) > 1 and sys.argv[1] == 'nets':
-        gen_net_step_cases()
+    if len(sys.argv) > 1 and sys.argv[1] in ('nets', 'generator'):
+        {'nets': gen_net_step_cases, 'generator': gen_generator_cases}[sys.argv[1]]()
         sys.exit(0)
     gen_loss_cases()
     gen_target_cases()
@@ -371,3 +388,4 @@ if __name__ == '__main__':
     gen_step_cases()
     gen_rnn_cases()
     gen_net_step_cases()
+    gen_generator_cases()

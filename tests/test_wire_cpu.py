@@ -13,7 +13,6 @@ from handyrl_b200.replay import DeviceReplay
 
 with open(os.path.join(GOLDEN, 'batch_cases.pkl'), 'rb') as f:
     CASES = pickle.load(f)
-REF = os.environ.get('HANDYRL_REFERENCE', '/root/reference')
 
 
 def same_flat(a, b):
@@ -49,29 +48,31 @@ def test_replay_accepts_both_formats():
         assert (getattr(a, k) == getattr(b, k)).all(), k
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'handyrl')), reason='reference checkout not mounted')
-def test_worker_hook_makes_the_reference_generator_ship_flat_episodes():
-    sys.path.insert(0, REF)
-    try:
-        import random
-        from handyrl.environment import make_env, prepare_env
-        from handyrl.generation import Generator
-        import handyrl.generation as gen
-        from handyrl.model import ModelWrapper
-        original = wire.install_worker_hook()
-        try:
-            env_args = {'env': 'TicTacToe'}
-            prepare_env(env_args)
-            env = make_env(env_args)
-            model = ModelWrapper(env.net())
-            random.seed(3)
-            ep = Generator(env, {'gamma': 0.8, 'compress_steps': 4}).generate({p: model for p in env.players()},
-                                                                              {'player': env.players(), 'model_id': {}})
-            assert ep is not None and 'flat' in ep and ep['steps'] == len(decode_moments(ep['moment']))
-            same_flat(wire.unpack_flat(ep['flat']), flatten_moments(decode_moments(ep['moment']), ep['outcome']))
-        finally:
-            gen.Generator.generate = original
-    finally:
-        sys.path.remove(REF)
-        for m in [m for m in sys.modules if m == 'handyrl' or m.startswith('handyrl.')]:
-            del sys.modules[m]
+def test_worker_hook_makes_the_reference_generator_ship_flat_episodes(monkeypatch):
+    """The hook wraps Generator.generate of an importable `handyrl.generation`; here that module is a stand-in whose
+    generate returns the episode the reference's own Generator produced (golden: generator_cases.pkl)."""
+    import copy
+    import types
+    with open(os.path.join(GOLDEN, 'generator_cases.pkl'), 'rb') as f:
+        golden = pickle.load(f)['tictactoe']
+
+    class Generator:
+        def __init__(self, env, args):
+            self.args = args
+
+        def generate(self, models, args):
+            return copy.deepcopy(golden['episode'])
+
+    gen = types.ModuleType('handyrl.generation')
+    gen.Generator = Generator
+    pkg = types.ModuleType('handyrl')
+    pkg.generation = gen
+    monkeypatch.setitem(sys.modules, 'handyrl', pkg)
+    monkeypatch.setitem(sys.modules, 'handyrl.generation', gen)
+    plain = Generator.generate
+    assert wire.install_worker_hook() is plain and Generator.generate is not plain
+    assert wire.install_worker_hook() is Generator.generate          # a second install does not wrap twice
+    ep = Generator(None, golden['args']).generate({}, golden['episode']['args'])
+    assert ep is not None and 'flat' in ep and ep['steps'] == len(decode_moments(ep['moment']))
+    assert ep['moment'] == golden['episode']['moment'] and ep['outcome'] == golden['episode']['outcome']
+    same_flat(wire.unpack_flat(ep['flat']), flatten_moments(decode_moments(ep['moment']), ep['outcome']))
